@@ -4,6 +4,8 @@
   python bench.py --gpus N --steps K --warmup W            (driver launches N>1 under torchrun)
   python bench.py --impl reference ...                     CPU arm: the oracle port of the reference's path
   python bench.py --config c4|c5 ...                       BASELINE configs[3] / [4]: engines sharing one lm:// server
+  python bench.py --dump-outputs DIR ...                   also write the last timed step's results as .npy files, so
+                                                           that two builds can be compared output for output
 
 Workload (N=1, default): BASELINE.json configs[1] -- a 32-layer / 32-head / 128-dim, 8192-token bf16 KV block (4 GiB),
 chunk_size 256 -> 32 chunks; every rank codes its own block (weak scaling, no data-path collective: the path shards by
@@ -38,6 +40,7 @@ sys.path.insert(0, ROOT)
 MODEL = "lmsys/longchat-7b-16k"
 L, H, D = 32, 32, 128
 C = H * D
+DUMP_SAMPLE = 1 << 22      # elements per array written by --dump-outputs: 16 MiB of float32 each
 
 
 def parse_args():
@@ -62,7 +65,16 @@ def parse_args():
                     help="container: rans_compact = v3 (default: rANS + symbol counts), rans = v2 (rANS + CDF rows), ac = v1")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (rank 0): the decoded "
+                         "KV and the last wave's container bytes as float32 (a fixed, seeded sample of each when larger "
+                         f"than {DUMP_SAMPLE} elements) and those containers' sizes as float64")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl, args.config) != ("b200", "c2"):
+        ap.error("--dump-outputs applies to the GPU arm's default workload (--impl b200 --config c2)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ synthetic data
@@ -201,7 +213,7 @@ def run_reference_arm(args):
     if rank != 0:
         return
     n = args.cpu_chunks
-    steps, warmup = max(3, min(args.steps, 5)), max(2, min(args.warmup, 3))
+    steps, warmup = args.steps, args.warmup
     gbs, (med, best), cores = cpu_codec_sample(n, args.chunk, steps, warmup)
     n_all = args.tokens // args.chunk
     sample = (f"{n} of {n_all} chunks ([{L},2,{args.chunk},{H},{D}] bf16 each) per step; median of {steps} steps after "
@@ -508,6 +520,9 @@ def main():
     barrier()
     ms_total = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        nw = sum(1 for _ in waves())
+        dump_outputs(args.dump_outputs, out, stagings[(nw - 1) % len(stagings)], stride, n_chunks - (nw - 1) * W, N)
     from lmcache_b200.dist_util import aggregate_gbps, max_over_ranks
     ms_step = max_over_ranks(ms_total, dev) / args.steps          # device time, max over ranks
     value = aggregate_gbps(raw_bytes, ms_step, world)              # weak scaling: every rank codes its own block
@@ -570,7 +585,7 @@ def main():
             step_device()
             sz = measure_sizes()
             par = parity_spot_check(kv, out, cs)
-            ms = timed(3)
+            ms = timed(args.steps)
             km = profile_kernels(2)
             sweep.append({"data": kind, "payload_bits_per_symbol": round(8.0 * (sum(sz) - n_chunks * fixed) / (raw_bytes / 2), 4),
                           "coder_bits_per_symbol": coder_bits(), "ms_per_step": round(ms, 4), "encode_ms": round(km.get("encode", 0), 4),
@@ -633,6 +648,30 @@ def staging_bytes(stride, W, N):
     return int(stride * W + N.READ_SLACK)
 
 
+def _sample(flat, n, seed):
+    """all of `flat` if it has at most n elements, else n of them at positions drawn from `seed` (the same every run)"""
+    import torch
+    if flat.numel() <= n:
+        return flat
+    idx = torch.randint(0, flat.numel(), (n,), generator=torch.Generator().manual_seed(seed))
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(dst, out, buf, stride, k, N):
+    """What the last timed step handed back: the decoded KV and the k containers of its last wave (found in `buf`,
+    `stride` bytes apart, each as long as its header's total_bytes)."""
+    import numpy as np
+    import torch
+    hdrs = buf[:k * stride].view(k, stride)[:, :N.HEADER_BYTES].cpu().numpy()
+    sizes = [int(N.Header.from_buffer_copy(hdrs[j].tobytes()).total_bytes) for j in range(k)]
+    containers = torch.cat([buf[j * stride:j * stride + s] for j, s in enumerate(sizes)])
+    os.makedirs(dst, exist_ok=True)
+    for name, a in (("decoded_kv", _sample(out.reshape(-1), DUMP_SAMPLE, 0).float()),
+                    ("containers", _sample(containers, DUMP_SAMPLE, 1).float()),
+                    ("container_sizes", torch.tensor(sizes, dtype=torch.float64))):
+        np.save(os.path.join(dst, name + ".npy"), a.cpu().numpy())
+
+
 def run_e2e(args, kv, dev, world, rank, barrier):
     """LMCacheEngine.store(tokens, kv) -> compressed page-locked host tier -> LMCacheEngine.retrieve(tokens), wall clock.
     No stream choreography here: the pipelines (encode || D2H, H2D || decode) live in the product
@@ -681,7 +720,7 @@ def run_e2e(args, kv, dev, world, rank, barrier):
     host_bytes = backend.host_bytes()
     cont_bytes = sum(e.nbytes for e in backend.dict.values() if e.blk is not None)
     barrier()
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
     t0 = time.perf_counter()
     parts = [one_step() for _ in range(steps)]
     barrier()
@@ -710,9 +749,9 @@ def run_e2e(args, kv, dev, world, rank, barrier):
         cur.synchronize()
         one_step(host_raw)
         t0 = time.perf_counter()
-        for _ in range(2):
+        for _ in range(steps):
             one_step(host_raw)
-        w2 = (time.perf_counter() - t0) / 2
+        w2 = (time.perf_counter() - t0) / steps
         host_raw.close()
         res["raw_upload_variant"] = {"value": round(raw_bytes / w2 / 1e9, 2), "unit": "GB/s", "ms_per_step": round(w2 * 1e3, 2),
                                      "h2d_bytes_per_step": raw_bytes + cont_bytes,

@@ -2,13 +2,15 @@
 process -- at the level that needs no GPU: token ids -> SHA-256 chain -> engine key strings -> B2KV containers over the
 wire -> header checks -> decode, with the CPU oracle standing in for the kernels on both sides;
 (2) wire interoperability with the REFERENCE's own server and client (lmcache/server/__main__.py:29-104,
-lmcache/storage_backend/connector/lm_connector.py:15-84), run from /root/reference with the import stubs of
-tests/_refstubs -- skipped where the reference tree is absent (the GPU box)."""
+lmcache/storage_backend/connector/lm_connector.py:15-84), through sessions recorded against them
+(tests/golden/golden_wire.json, made by tests/golden/make_wire_golden.py)."""
 import ctypes
+import json
 import os
 import socket
 import subprocess
 import sys
+import threading
 import time
 
 import numpy as np
@@ -16,7 +18,6 @@ import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-REF = "/root/reference"
 
 
 def _free_port():
@@ -116,46 +117,113 @@ def test_c4_flow_two_processes_one_server(coder, server_kind, tmp_path):
         srv.wait()
 
 
-needs_ref = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "lmcache")), reason="reference tree not present (GPU box)")
+def _our_client_blobs():
+    rng = np.random.default_rng(5)
+    return {f"vllm@lmsys/longchat-7b-16k@2@0@{i:064x}": rng.integers(0, 256, n, dtype=np.uint8).tobytes()
+            for i, n in enumerate([1, 157, 65536, 2 * 1024 * 1024 + 3])}
 
 
-@needs_ref
+def _reference_client_blobs():
+    return {"vllm@a/b@1@0@" + "%064x" % i: bytes([i]) * n for i, n in enumerate([1, 158, 70000, 1 << 21])}
+
+
+def _our_client_session(c, blobs):
+    """set / exists / get / get_into / miss / list through one of this package's clients (also what
+    tests/golden/make_wire_golden.py ran against the reference server)"""
+    for k, v in blobs.items():
+        c.set(k, v)
+    for k, v in blobs.items():
+        for _ in range(400):
+            if c.exists(k):
+                break
+            time.sleep(0.005)
+        assert c.exists(k)
+        assert bytes(c.get(k)) == v
+        buf = np.zeros(len(v) + 64, np.uint8)
+        assert c.get_into(k, buf.ctypes.data, buf.size) == len(v) and buf[:len(v)].tobytes() == v
+    assert not c.exists("vllm@m@1@0@" + "f" * 64) and c.get("vllm@m@1@0@" + "f" * 64) is None
+    assert sorted(c.list()) == sorted(blobs)
+    c.close()
+
+
+def _transcript(name):
+    """frames of a session recorded against the reference's own server (tests/golden/make_wire_golden.py)"""
+    return json.load(open(os.path.join(HERE, "golden", "golden_wire.json")))[name]
+
+
+def _frame_bytes(f, blobs):
+    if "hex" in f:
+        return bytes.fromhex(f["hex"])
+    if "blob" in f:
+        return blobs[f["blob"]]
+    return "\n".join(f["keys"]).encode()
+
+
+def _recv_exact(s, n):
+    buf = bytearray()
+    while len(buf) < n:
+        k = s.recv(n - len(buf))
+        if not k:
+            raise AssertionError(f"connection closed after {len(buf)} of {n} bytes")
+        buf += k
+    return bytes(buf)
+
+
+class _ReferenceServerReplay:
+    """Plays the reference server's side of a recorded session to ONE client: every byte the client sends must be the
+    byte the reference server received, and the client gets the reference server's replies verbatim."""
+
+    def __init__(self, frames, blobs):
+        self.lsock = socket.socket()
+        self.lsock.bind(("127.0.0.1", 0))
+        self.lsock.listen(1)
+        self.lsock.settimeout(60)
+        self.port = self.lsock.getsockname()[1]
+        self.frames, self.blobs, self.error = frames, blobs, None
+        self.thread = threading.Thread(target=self._run, daemon=True)
+        self.thread.start()
+
+    def _run(self):
+        try:
+            cli, _ = self.lsock.accept()
+            cli.settimeout(60)
+            with cli:
+                for i, f in enumerate(self.frames):
+                    want = _frame_bytes(f, self.blobs)
+                    if f["from"] == "server":
+                        cli.sendall(want)
+                    else:
+                        got = _recv_exact(cli, len(want))
+                        assert got == want, f"frame {i}: the client sent {got[:200]!r}, the reference server received {want[:200]!r}"
+                assert cli.recv(1) == b"", "the client sent more than the recorded session"
+        except BaseException as e:       # noqa: BLE001 -- reported by join() on the test's thread
+            self.error = e
+        finally:
+            self.lsock.close()
+
+    def join(self):
+        self.thread.join(120)
+        assert not self.thread.is_alive(), "replay server still waiting for the client"
+        if self.error is not None:
+            raise self.error
+
+
 @pytest.mark.parametrize("scheme", ["lm", "lmn"])
 def test_our_clients_against_the_reference_server(scheme):
-    """python -m lmcache.server from /root/reference, driven by this package's two lm:// clients"""
+    """This package's two lm:// clients against the reference's `python -m lmcache.server`, replayed from a recorded
+    session: requests byte-identical to what that server accepted, its replies understood."""
     from lmcache_b200.storage_backend.connector import CreateConnector
-    port = _free_port()
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(HERE, "_refstubs"), REF]))
-    srv = subprocess.Popen([sys.executable, "-m", "lmcache.server", "127.0.0.1", str(port)], env=env, cwd="/tmp",
-                           stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    blobs = _our_client_blobs()
+    srv = _ReferenceServerReplay(_transcript("our_clients"), list(blobs.values()))
     try:
-        assert _wait_port(port, srv), "reference server did not start"
-        c = CreateConnector(f"{scheme}://127.0.0.1:{port}")
-        rng = np.random.default_rng(5)
-        blobs = {f"vllm@lmsys/longchat-7b-16k@2@0@{i:064x}": rng.integers(0, 256, n, dtype=np.uint8).tobytes()
-                 for i, n in enumerate([1, 157, 65536, 2 * 1024 * 1024 + 3])}
-        for k, v in blobs.items():
-            c.set(k, v)
-        for k, v in blobs.items():
-            for _ in range(400):
-                if c.exists(k):
-                    break
-                time.sleep(0.005)
-            assert c.exists(k)
-            assert bytes(c.get(k)) == v
-            buf = np.zeros(len(v) + 64, np.uint8)
-            assert c.get_into(k, buf.ctypes.data, buf.size) == len(v) and buf[:len(v)].tobytes() == v
-        assert not c.exists("vllm@m@1@0@" + "f" * 64) and c.get("vllm@m@1@0@" + "f" * 64) is None
-        assert sorted(c.list()) == sorted(blobs)
-        c.close()
+        _our_client_session(CreateConnector(f"{scheme}://127.0.0.1:{srv.port}"), blobs)
     finally:
-        srv.terminate()
-        srv.wait()
+        srv.join()
 
 
-@needs_ref
 def test_reference_client_against_our_native_server():
-    """the reference's LMCServerConnector (imported from /root/reference in a subprocess) against csrc/lmnet.cu's server"""
+    """The reference's LMCServerConnector against csrc/lmnet.cu's server: the requests that client sent in a recorded
+    session go to our server, whose replies must be the reference server's (LIST: the same keys, in any order)."""
     import __graft_entry__ as ge
     ge.build_cuda()
     from lmcache_b200 import _native as N
@@ -163,27 +231,19 @@ def test_reference_client_against_our_native_server():
     h = ctypes.c_void_p()
     N.check(lib.b200kv_lm_server_start(b"127.0.0.1", 0, ctypes.byref(h)))
     port = lib.b200kv_lm_server_port(h)
-    code = f'''
-import sys, time
-sys.path[:0] = [{os.path.join(HERE, "_refstubs")!r}, {REF!r}]
-from lmcache.storage_backend.connector.lm_connector import LMCServerConnector
-c = LMCServerConnector("127.0.0.1", {port})
-blobs = {{"vllm@a/b@1@0@" + "%064x" % i: bytes([i]) * n for i, n in enumerate([1, 158, 70000, 1 << 21])}}
-for k, v in blobs.items():
-    c.set(k, v)
-for k, v in blobs.items():
-    for _ in range(400):
-        if c.exists(k): break
-        time.sleep(0.005)
-    assert c.exists(k) and bytes(c.get(k)) == v, k
-assert not c.exists("nope@x@1@0@00") and c.get("nope@x@1@0@00") is None
-assert sorted(c.list()) == sorted(blobs)
-c.close()
-print("ok")
-'''
+    blobs = list(_reference_client_blobs().values())
     try:
-        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=120, cwd="/tmp")
-        assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stderr[-3000:]
+        with socket.create_connection(("127.0.0.1", port), timeout=60) as s:
+            for i, f in enumerate(_transcript("reference_client")):
+                want = _frame_bytes(f, blobs)
+                if f["from"] == "client":
+                    s.sendall(want)
+                    continue
+                got = _recv_exact(s, len(want))
+                if "keys" in f:
+                    assert sorted(got.decode().split("\n")) == sorted(f["keys"]), f"frame {i}: LIST"
+                else:
+                    assert got == want, f"frame {i}: our server replied {got[:200]!r}, the reference server {want[:200]!r}"
         assert lib.b200kv_lm_server_num_keys(h) == 4
     finally:
         N.check(lib.b200kv_lm_server_stop(h))
